@@ -1,6 +1,6 @@
 """bench.py — samples/sec of the DLRM-Criteo train step (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path over one synthetic Criteo batch: KJT scan -> (bucketize + all-to-all at
 N>1) -> pooled gather -> DLRM dot interaction + dense towers -> BCE loss -> backward with the fused sparse
@@ -95,7 +95,15 @@ def parse_args():
                     help="N>1: skip the in-process parity check of the sharded step against its unsharded twin")
     ap.add_argument("--force-sharded", action="store_true",
                     help="N=1 only: still go through bucketize / all-to-all / owner gather (1-rank process group)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps: what the last timed step left for its caller (loss, dense parameters, "
+                         "a fixed sample of rows of every table and of its optimizer state) as DIR/<name>.npy, float32")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus > 1 or args.force_sharded):
+        ap.error("--dump-outputs: single-GPU unsharded runs of --impl ours only")
+    return args
 
 
 class ClockSampler:
@@ -373,10 +381,12 @@ def run_ours(args):
     e0.record()
     for i in range(K):
         step.load(ring[i % len(ring)])
-        step.replay()
+        loss = step.replay()
     e1.record()
     barrier()
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs:      # before anything below steps the model again
+        dump_outputs(args.dump_outputs, pipe, loss)
     # ---- e2e: pinned host batch -> H2D -> step -> loss back on the host, every step --------------------------
     # The H2D of batch i+1 runs on the copy stream while step i computes (graphed steps); the loss of EVERY step
     # reaches the host inside the timed region through a pinned D2H copy + event, read one step later so that the
@@ -583,6 +593,44 @@ def run_ours(args):
             extras["e2e_blocking"] = {"failed": repr(e)[:200]}
         args._extras = extras
     _emit(args, world, B, K, W, ms_total, ms_e2e, host, last, launches_per_step, clk, roofline, cpu, len(ring))
+
+
+DUMP_ROWS_PER_TABLE = 4096
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, pipe, loss: torch.Tensor) -> None:
+    """Writes what a train step hands its caller, as of the last timed step: the loss and the model it updated — every
+    dense parameter in full and, of every embedding table, the weights and optimizer state of a fixed sample of rows
+    (all rows of a table up to DUMP_ROWS_PER_TABLE rows; otherwise that many draws of a generator seeded per table)."""
+    import numpy as np
+
+    out = {"loss": loss.detach().reshape(1)}
+    dense = {id(p) for p in pipe.model.dense_parameters()}
+    for name, p in pipe.model.named_parameters():
+        if id(p) in dense:
+            out[f"dense.{name}"] = p.detach()
+    for c, coll in enumerate(pipe.model.sparse_collections()):
+        for t in sorted(coll._table_off):
+            n_rows = coll._table_rows[t]
+            if n_rows <= DUMP_ROWS_PER_TABLE:
+                rows = torch.arange(n_rows)
+            else:
+                gen = torch.Generator().manual_seed(1000 * c + t)
+                rows = torch.randint(n_rows, (DUMP_ROWS_PER_TABLE,), generator=gen).unique()
+            rows = rows.to(coll.weights.device)
+            name = f"sparse{c}.{coll._configs[t].name}"
+            out[f"{name}.weight"] = coll.table_weight(t).index_select(0, rows)
+            state = coll.table_state(t)
+            if state is not None:
+                out[f"{name}.state"] = state.index_select(0, rows)
+    arrays = {k: v.float().cpu().numpy() for k, v in out.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a.astype(np.float32, copy=False))
 
 
 def _peer_roofline(pipe, kern, ring, B, world, iters, step_ms):

@@ -1,12 +1,16 @@
-"""Generates golden vectors from the REFERENCE's own modules (run in the build container only).
+"""Generates golden vectors from a checkout of the reference project (alibaba/TorchEasyRec @ 54cac316).
 
 The reference package cannot be imported as a whole (torchrec / fbgemm_gpu / pyfg are absent), but
 tzrec/modules/fm.py, interaction.py, mlp.py, mmoe.py, task_tower.py and sequence.py are plain PyTorch: they are loaded file by file
 through stub parent packages, executed on seeded inputs, and their outputs (and autograd gradients) are
-stored as small .npz fixtures.  /root/reference does not travel to the GPU box; the fixtures do.
+stored as small .npz fixtures.  `configs` stores what this project's config loader makes of every examples/*.config.
+The tests read only the fixtures, so they run without the reference checkout.
 
-    python tests/golden/make_golden_from_reference.py [dense|blocks]
+    python tests/golden/make_golden_from_reference.py <reference checkout> [dense|blocks|configs]
 """
+import glob
+import gzip
+import json
 import os
 import sys
 import types
@@ -14,7 +18,7 @@ import types
 import numpy as np
 import torch
 
-REF = "/root/reference"
+REF = ""     # the reference checkout, set from the command line
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -119,39 +123,51 @@ def main():
         z.backward(dz)
         out[f"{tag}_x"], out[f"{tag}_z"], out[f"{tag}_dz"], out[f"{tag}_dx"] = (
             x.detach().numpy(), z.detach().numpy(), dz.numpy(), x.grad.numpy())
-    # DLRM predict glue (tzrec/models/dlrm.py:113-131) re-enacted with the reference modules
+    # DLRM predict glue (tzrec/models/dlrm.py:113-131) re-enacted with the reference modules, forward only
     B, Ns, D = 32, 26, 16
     dense_mlp = MLP(13, [64, 16])
     final_mlp = MLP(351 + 16 + Ns * D, [64, 32])
     head = torch.nn.Linear(32, 1)
     dense_in = torch.rand(B, 13)
-    sparse = torch.randn(B, Ns * D, requires_grad=True)
-    dense_feat = dense_mlp(dense_in)
-    feat = torch.cat([dense_feat.unsqueeze(1), sparse.reshape(-1, Ns, D)], dim=1)
-    inter = InteractionArch(Ns + 1)(feat)
-    all_feat = torch.cat([inter, dense_feat, sparse], dim=-1)
-    logits = head(final_mlp(all_feat)).squeeze(1)
-    labels = (torch.rand(B) < 0.25).float()
-    loss = torch.nn.functional.binary_cross_entropy_with_logits(logits, labels)
-    loss.backward()
-    out["dlrm_dense_in"], out["dlrm_sparse"], out["dlrm_labels"] = dense_in.numpy(), sparse.detach().numpy(), labels.numpy()
-    out["dlrm_all_feat"], out["dlrm_logits"], out["dlrm_loss"] = all_feat.detach().numpy(), logits.detach().numpy(), loss.detach().numpy()
-    out["dlrm_dsparse"] = sparse.grad.numpy()
-    sd = {}
+    sparse = torch.randn(B, Ns * D)
+    with torch.no_grad():
+        dense_feat = dense_mlp(dense_in)
+        feat = torch.cat([dense_feat.unsqueeze(1), sparse.reshape(-1, Ns, D)], dim=1)
+        inter = InteractionArch(Ns + 1)(feat)
+        all_feat = torch.cat([inter, dense_feat, sparse], dim=-1)
+        logits = head(final_mlp(all_feat)).squeeze(1)
+        labels = (torch.rand(B) < 0.25).float()
+        loss = torch.nn.functional.binary_cross_entropy_with_logits(logits, labels)
+    out["dlrm_dense_in"], out["dlrm_sparse"], out["dlrm_labels"] = dense_in.numpy(), sparse.numpy(), labels.numpy()
+    out["dlrm_all_feat"], out["dlrm_logits"], out["dlrm_loss"] = all_feat.numpy(), logits.numpy(), loss.numpy()
     for prefix, mod in [("dense_mlp", dense_mlp), ("final_mlp", final_mlp), ("output_mlp", head)]:
         for k, v in mod.state_dict().items():
-            sd[f"dlrm_sd__{prefix}.{k}"] = v.numpy()
-        for k, p in mod.named_parameters():
-            sd[f"dlrm_grad__{prefix}.{k}"] = p.grad.numpy()
-    out.update(sd)
+            out[f"dlrm_sd__{prefix}.{k}"] = v.numpy()
     np.savez_compressed(os.path.join(HERE, "ref_dense_modules.npz"), **out)
     print("wrote", os.path.join(HERE, "ref_dense_modules.npz"), len(out), "arrays")
 
 
+def example_configs():
+    """Every examples/*.config of the reference as this project's loader parses it (`Message.to_dict()`), keyed by
+    file name -> tests/golden/reference_example_configs.json.gz."""
+    sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+    from torcheasyrec_b200.config import load_pipeline_config
+
+    out = {os.path.basename(p)[:-len(".config")]: load_pipeline_config(p).to_dict()
+           for p in sorted(glob.glob(os.path.join(REF, "examples", "*.config")))}
+    path = os.path.join(HERE, "reference_example_configs.json.gz")
+    with gzip.GzipFile(path, "wb", mtime=0) as fh:
+        fh.write(json.dumps(out, indent=1, sort_keys=True).encode())
+    print("wrote", path, len(out), "configs")
+
+
 if __name__ == "__main__":
-    which = sys.argv[1] if len(sys.argv) > 1 else "all"
+    REF = os.path.abspath(sys.argv[1])
+    which = sys.argv[2] if len(sys.argv) > 2 else "all"
     if which in ("all", "dense"):
         main()
     if which in ("all", "blocks"):
         _stub_packages()
         model_blocks()
+    if which in ("all", "configs"):
+        example_configs()

@@ -1,5 +1,9 @@
-"""Config surface: the reference's examples/*.config load unchanged, and the generated configs are equivalent."""
-import glob
+"""Config surface: the reference's examples/*.config load unchanged, and the generated configs are equivalent.
+
+The reference's examples are represented by tests/golden/reference_example_configs.json.gz: what `load_pipeline_config`
+made of each of them (`to_dict()`), written by tests/golden/make_golden_from_reference.py (`configs`)."""
+import gzip
+import json
 import os
 
 import pytest
@@ -8,26 +12,30 @@ from torcheasyrec_b200 import example_configs
 from torcheasyrec_b200.config import config_to_kwargs, edit_config, load_pipeline_config, parse_text
 from torcheasyrec_b200.features import create_features
 
-REF_EXAMPLES = "/root/reference/examples"
-have_ref = pytest.mark.skipif(not os.path.isdir(REF_EXAMPLES), reason="reference checkout not present (GPU box)")
+with gzip.open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden",
+                            "reference_example_configs.json.gz"), "rt") as _fh:
+    REF_EXAMPLES = json.load(_fh)
 
 
-@have_ref
-def test_all_reference_examples_parse():
-    files = sorted(glob.glob(os.path.join(REF_EXAMPLES, "*.config")))
-    assert len(files) >= 17
-    for p in files:
-        cfg = load_pipeline_config(p)
-        assert cfg.model_config.WhichOneof("model") is not None, p
+def _reference_example(name, tmp_path):
+    """The reference's examples/<name>.config as a pipeline config file (the JSON form the loader also accepts)."""
+    path = tmp_path / (name + ".json")
+    path.write_text(json.dumps(REF_EXAMPLES[name]))
+    return str(path)
+
+
+def test_all_reference_examples_parse(tmp_path):
+    assert len(REF_EXAMPLES) >= 17
+    for name in REF_EXAMPLES:
+        cfg = load_pipeline_config(_reference_example(name, tmp_path))
+        assert cfg.model_config.WhichOneof("model") is not None, name
         assert len(cfg.feature_configs) > 0
 
 
-@have_ref
 @pytest.mark.parametrize("name", list(example_configs.GENERATORS))
 def test_generated_config_equals_reference_example(name):
-    ref = load_pipeline_config(os.path.join(REF_EXAMPLES, name + ".config"))
     ours = parse_text(example_configs.GENERATORS[name]())
-    assert ours.to_dict() == ref.to_dict()
+    assert ours.to_dict() == REF_EXAMPLES[name]
 
 
 @pytest.mark.parametrize("name,groups", [
@@ -93,13 +101,12 @@ def test_sparse_optimizer_mapping_from_train_config():
     assert s.kind == OPT_PARTIAL_ROWWISE_ADAM and s.max_gradient == 0.0
 
 
-@have_ref
 @pytest.mark.parametrize("name", ["dlrm_criteo", "deepfm_criteo", "mmoe_taobao", "multi_tower_din_taobao",
                                   "multi_tower_taobao"])
-def test_reference_example_config_runs_unchanged(name):
-    """north_star: `examples/*.config` runs unchanged — the reference's own file is loaded from its checkout (only the
-    table sizes are capped, like the reference's --edit_config_json), the model is built and stepped twice on the CPU
-    with the oracle as compute; the loss must be finite and move."""
+def test_reference_example_config_runs_unchanged(name, tmp_path):
+    """north_star: `examples/*.config` runs unchanged — the reference's own example is loaded (only the table sizes
+    are capped, like the reference's --edit_config_json), the model is built and stepped twice on the CPU with the
+    oracle as compute; the loss must be finite and move."""
     import sys
 
     import torch
@@ -110,7 +117,7 @@ def test_reference_example_config_runs_unchanged(name):
     from torcheasyrec_b200 import functional as Fn
     from torcheasyrec_b200.engine import Pipeline
 
-    pipe = Pipeline(os.path.join(REF_EXAMPLES, name + ".config"), device="cpu", max_rows=200, seed=3)
+    pipe = Pipeline(_reference_example(name, tmp_path), device="cpu", max_rows=200, seed=3)
     batch = pipe.synthetic_batch(24, seed=1)
     with Fn.use_backend(OracleKernels()):
         l0 = float(pipe.eager_step(batch))
